@@ -2,7 +2,7 @@
 """bench.py — VOLDOR EM hot path on B200.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|cpu-port|abi-dropin]
-                  [--inflight M] [--no-extras] [--no-cpu-baseline]
+                  [--inflight M] [--no-extras] [--no-cpu-baseline] [--dump-outputs DIR]
 
 Workload (both arms, `config.workload`): BASELINE.json configs[1] — a single 640x480 frame with 8 flows, 30 EM
 iterations, monocular (bootstrap pose/depth injected, BASELINE.md §3), 8192 pose hypotheses per camera, window
@@ -29,6 +29,10 @@ all_gather per step; "scaling": "weak".
              (oracle/_ref) run on the same input from the same fresh state
   extra : the other single-GPU BASELINE configs (C1 with the CPU restatement timed beside it, C3, C5), one window in
           flight, each with its own roofline figures
+
+--dump-outputs DIR writes what the last timed step returned for each window in flight (rank 0), as float32
+DIR/ctx<k>_{poses,poses_covar,depth,depth_conf}.npy: the arrays voldor() returns, poses cut to the registered frames.
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 --impl reference runs the REFERENCE arm: the reference's own CUDA kernels (oracle/_ref, its unmodified .cu files
 rebuilt for sm_100a) driven by the reference's host orchestration restated OpenCV-free over the ABI
@@ -305,6 +309,7 @@ class WindowRunner:
         pageable (numpy buffers through the reference-facing C++ symbol py_voldor_wrapper)"""
         self.lib.vb_context_select(self.ctx)
         n, it = C.c_int(0), C.c_int(0)
+        self.n_registered = None
         stats = np.zeros(4, np.float32)
         p = self._p
         if mode == "pageable":
@@ -313,6 +318,7 @@ class WindowRunner:
                 p(i["flows"]), p(i["disparity"]), None, p(i["depth_priors"]), p(i["depth_prior_poses"]), None,
                 *map(C.c_float, self.f), C.c_float(self.basefocal), self.N, self.N_dp, self.w, self.h, self.cfg,
                 C.byref(n), p(o["poses"]), p(o["covar"]), p(o["depth"]), p(o["conf"]))
+            self.n_registered = n.value
             return n.value, int(self.cfg.split(b"--max_iters ")[1].split()[0]), stats
         i = self.dev_in if mode == "resident" else self.pin_in
         depth = self.out_d["depth"] if mode == "resident" else self.out_h["depth"]
@@ -322,6 +328,7 @@ class WindowRunner:
                                          C.c_float(self.basefocal), self.N, self.N_dp, self.w, self.h, self.cfg,
                                          C.byref(n), p(self.out_h["poses"]), p(self.out_h["covar"]), p(depth), p(conf),
                                          C.byref(it), stats.ctypes.data_as(FP))
+        self.n_registered = n.value
         return n.value, it.value, stats
 
     def outputs(self, mode):
@@ -334,6 +341,17 @@ class WindowRunner:
         d = self.out_d if mode == "resident" else self.out_h
         return {"poses": self.out_h["poses"].numpy().copy(), "covar": self.out_h["covar"].numpy().copy(),
                 "depth": d["depth"].cpu().numpy().copy(), "conf": d["conf"].cpu().numpy().copy()}
+
+
+def dump_outputs(path, runners, mode):
+    """the outputs of the last window each runner solved in `mode`, as voldor() hands them to its caller"""
+    os.makedirs(path, exist_ok=True)
+    for r in runners:
+        o, n = r.outputs(mode), r.n_registered
+        arrays = {"poses": o["poses"][:n], "poses_covar": o["covar"][:n].reshape(n, 6, 6), "depth": o["depth"],
+                  "depth_conf": o["conf"]}
+        for name, a in arrays.items():
+            np.save(os.path.join(path, f"ctx{r.ctx}_{name}.npy"), np.ascontiguousarray(a, np.float32))
 
 
 class ContextWorkers:
@@ -527,6 +545,8 @@ def bench_ours(args, rank, world, local_rank):
     clocks = ClockSampler(local_rank) if rank == 0 else None
     ms_res, iters_res, frames_res, lat_res = timed("resident", args.steps, args.warmup, clocks)
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, runners, "resident")
     ms_e2e, iters_e2e, _, lat_e2e = timed("pinned", args.steps, max(1, args.warmup // 2))
 
     # the collective really carried this rank's poses (C4 identity of the exchange)
@@ -678,6 +698,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", dest="no_cpu_baseline", action="store_true")
     ap.add_argument("--no-extras", dest="no_extras", action="store_true")
     ap.add_argument("--no-parity", dest="no_parity", action="store_true")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as float32 .npy files into DIR")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
 

@@ -38,6 +38,10 @@
 
 #ifdef HAVE_REF_LAMBDATWIST
 #include "lambdatwist/lambdatwist_p4p.h"
+#else
+// without the reference checkout: the product's lambda-twist lanes, built for the host (individually rounded operations,
+// the same hypotheses bit for bit as the reference kernels: tests/test_cpu_p3p_quad.py)
+#include "../voldor_b200/csrc/p3p_twist_quad.cuh"
 #endif
 
 namespace {
@@ -498,9 +502,33 @@ int cpu_solve_batch_p3p_lambdatwist_gpu(float* h_p3s, float* h_p2s, float* o_rve
     }
     return 0;
 #else
-    (void)h_p3s, (void)h_p2s, (void)o_rvecs, (void)o_tvecs, (void)h_K, (void)N_pts, (void)N_poses;
-    printf("oracle: built without the reference lambdatwist headers\n");
-    return 1;
+    const float fx = h_K[0], cx = h_K[2], fy = h_K[4], cy = h_K[5];
+#pragma omp parallel for schedule(dynamic, 64)
+    for (int idx = 0; idx < N_poses; idx++) {
+        curandStateXORWOW_t st;
+        curand_init(233ULL, (unsigned long long)idx, 0ULL, &st);
+        float uv[8];
+        vb::quad::Vec3f X[4];
+        for (int k = 0; k < 4; k++) {
+            const int i = std::min((int)(curand_uniform(&st) * N_pts), N_pts - 1);
+            uv[2 * k] = h_p2s[2 * i], uv[2 * k + 1] = h_p2s[2 * i + 1];
+            X[k] = vb::quad::Vec3f{h_p3s[3 * i], h_p3s[3 * i + 1], h_p3s[3 * i + 2]};
+        }
+        vb::quad::Pose P[4];
+        bool exists[4];
+        float err[4];
+        for (int q = 0; q < 4; q++) err[q] = 0.f, exists[q] = vb::quad::twist_lane(q, uv, X, fx, fy, cx, cy, P[q], err[q]);
+        const int best = vb::quad::pick_by_fourth_point(exists, err);
+        float* rv = o_rvecs + idx * 3;
+        float* tv = o_tvecs + idx * 3;
+        if (best < 0) {
+            rv[0] = rv[1] = rv[2] = tv[0] = tv[1] = tv[2] = NAN;
+            continue;
+        }
+        tv[0] = P[best].t[0], tv[1] = P[best].t[1], tv[2] = P[best].t[2];
+        vb::hm::matrix_to_rvec(P[best].R, rv);
+    }
+    return 0;
 #endif
 }
 int cpu_solve_batch_p3p_ap3p_gpu(float* a, float* b, float* c, float* d, float* e, int n, int m) {

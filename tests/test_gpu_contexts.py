@@ -9,6 +9,7 @@ import pytest
 
 import ffi
 import oracle_host
+import refgold
 import synth
 import voldor_b200
 
@@ -55,12 +56,16 @@ def test_concurrent_contexts_each_equal_a_fresh_reference_process():
     [t.start() for t in ts]
     [t.join() for t in ts]
     assert not errors, errors
-    for k in series:
+
+    def reference_process(k):
         ref_lib = oracle_host.fresh_reference_copy(f"ctx{k}")
         ffi.libc_srand(50 + k)
-        for j, (win, boot) in enumerate(series[k]):
-            ref = oracle_host.run_window(ref_lib, win["flows"], win["fx"], win["fy"], win["cx"], win["cy"], config=CFG,
-                                         boot=boot)
+        return [oracle_host.run_window(ref_lib, win["flows"], win["fx"], win["fy"], win["cx"], win["cy"], config=CFG,
+                                       boot=boot) for win, boot in series[k]]
+
+    for k in series:
+        refs = refgold.reference(lambda: reference_process(k))
+        for j, ref in enumerate(refs):
             got = mine[k][j]
             assert got["n_registered"] == ref["n_registered"] > 0 and got["iters"] == ref["iters"]
             for key in ("poses", "poses_covar", "depth", "depth_conf"):
@@ -100,7 +105,8 @@ def test_context_zero_unaffected_by_other_contexts():
         stop.set()
         [t.join() for t in ts]
     ffi.libc_srand(3)
-    ref = oracle_host.run_window(oracle_host.fresh_reference_copy("solo"), *args, config=CFG, boot=boot)
+    ref = refgold.reference(
+        lambda: oracle_host.run_window(oracle_host.fresh_reference_copy("solo"), *args, config=CFG, boot=boot))
     for key in ("poses", "poses_covar", "depth", "depth_conf"):
         assert ffi.bits_equal(a[key], ref[key]), key
 

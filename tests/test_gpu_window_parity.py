@@ -9,11 +9,17 @@ import pytest
 
 import ffi
 import oracle_host
+import refgold
 import synth
 import voldor_b200
 
 pytestmark = pytest.mark.gpu
 OUT = os.path.join(ffi.ROOT, "gpurun_out")
+
+
+@pytest.fixture(autouse=True)
+def _fresh_depth_rng():
+    refgold.reseed_depth_rng()
 
 
 def _report(rep):
@@ -52,13 +58,13 @@ def test_mono_window_bit_exact(w, h, N, iters):
     # resident path share one stream, so the three series are interleaved to keep both libraries at the same
     # point of their history: (ref#1, ours-abi#1) then (ref#2, ours-resident#2).
     ffi.libc_srand(77)
-    ref1 = oracle_host.run_window("ref", *args, config=cfg, boot=boot)
+    ref1 = refgold.reference(lambda: oracle_host.run_window("ref", *args, config=cfg, boot=boot))
     ffi.libc_srand(77)
     abi1 = oracle_host.run_window("ours_abi", *args, config=cfg, boot=boot)
     assert ref1["n_registered"] == N
     _compare(f"window mono {w}x{h}x{N} abi-vs-ref", abi1, ref1)
     ffi.libc_srand(78)
-    ref2 = oracle_host.run_window("ref", *args, config=cfg, boot=boot)
+    ref2 = refgold.reference(lambda: oracle_host.run_window("ref", *args, config=cfg, boot=boot))
     voldor_b200.set_bootstrap_override(*boot)
     ffi.libc_srand(78)
     mine2 = voldor_b200.voldor_ex(*args, config=cfg)
@@ -76,7 +82,7 @@ def test_prior_window_bit_exact():
     args = (win["flows"], win["fx"], win["fy"], win["cx"], win["cy"])
     kw = dict(depth_priors=prior, depth_prior_poses=pose, config=cfg)
     ffi.libc_srand(5)
-    ref = oracle_host.run_window("ref", *args, **kw)
+    ref = refgold.reference(lambda: oracle_host.run_window("ref", *args, **kw))
     ffi.libc_srand(5)
     mine = voldor_b200.voldor_ex(*args, **kw)
     assert ref["n_registered"] > 0
@@ -95,7 +101,7 @@ def test_disparity_window_bit_exact():
     args = (win["flows"], win["fx"], win["fy"], win["cx"], win["cy"])
     kw = dict(basefocal=basefocal, disparity=disp, config=cfg)
     ffi.libc_srand(6)
-    ref = oracle_host.run_window("ref", *args, **kw)
+    ref = refgold.reference(lambda: oracle_host.run_window("ref", *args, **kw))
     ffi.libc_srand(6)
     mine = voldor_b200.voldor_ex(*args, **kw)
     assert ref["n_registered"] > 0
@@ -145,7 +151,7 @@ def test_baseline_config_shapes_bit_exact(name, w, h, N, iters, poses, kind):
     else:
         kw.update(depth_priors=synth.noisy_depth(win, 0.01)[None], depth_prior_poses=np.zeros((1, 6), np.float32))
     ffi.libc_srand(9)
-    ref = oracle_host.run_window("ref", *args, boot=boot, **kw)
+    ref = refgold.reference(lambda: oracle_host.run_window("ref", *args, boot=boot, **kw))
     if boot:
         voldor_b200.set_bootstrap_override(*boot)
     ffi.libc_srand(9)
@@ -163,7 +169,7 @@ def test_c2_benchmarked_configuration_30_iterations_bit_exact():
     win, boot = bench.make_inputs(0)
     args = (win["flows"], win["fx"], win["fy"], win["cx"], win["cy"])
     ffi.libc_srand(1000)
-    ref = oracle_host.run_window("ref", *args, config=bench.CONFIG, boot=boot)
+    ref = refgold.reference(lambda: oracle_host.run_window("ref", *args, config=bench.CONFIG, boot=boot))
     voldor_b200.set_bootstrap_override(*boot)
     ffi.libc_srand(1000)
     mine = voldor_b200.voldor_ex(*args, config=bench.CONFIG)
@@ -182,7 +188,7 @@ def test_benchmarked_extra_configurations_full_iterations_bit_exact(name):
     assert boot is None
     args = (win["flows"], win["fx"], win["fy"], win["cx"], win["cy"])
     ffi.libc_srand(2000)
-    ref = oracle_host.run_window("ref", *args, config=cfg, **kw)
+    ref = refgold.reference(lambda: oracle_host.run_window("ref", *args, config=cfg, **kw))
     ffi.libc_srand(2000)
     mine = voldor_b200.voldor_ex(*args, config=cfg, **kw)
     c = bench.CASES[name]
@@ -198,7 +204,7 @@ def test_c1_configuration_bit_exact():
     cfg = f"--silent --max_iters {iters} --no_trunc_iters 1000 --n_poses_to_sample 8192"
     args = (win["flows"], win["fx"], win["fy"], win["cx"], win["cy"])
     ffi.libc_srand(12)
-    ref = oracle_host.run_window("ref", *args, config=cfg, boot=boot)
+    ref = refgold.reference(lambda: oracle_host.run_window("ref", *args, config=cfg, boot=boot))
     voldor_b200.set_bootstrap_override(*boot)
     ffi.libc_srand(12)
     mine = voldor_b200.voldor_ex(*args, config=cfg)
@@ -233,10 +239,13 @@ def test_vo_sequence_chained_windows_bit_exact():
         outs["mine"].append(r)
         return r
 
-    ffi.libc_srand(31)
-    vo_ref = vo_frontend.VisualOdometry(win["fx"], win["fy"], win["cx"], win["cy"], winsize=4, user_config=user,
-                                        solver=ref_solver)
-    T_ref = vo_ref.run(list(win["flows"]))
+    def run_ref():
+        ffi.libc_srand(31)
+        vo_ref = vo_frontend.VisualOdometry(win["fx"], win["fy"], win["cx"], win["cy"], winsize=4, user_config=user,
+                                            solver=ref_solver)
+        return vo_ref.run(list(win["flows"])), outs["ref"]
+
+    T_ref, outs["ref"] = refgold.reference(run_ref)
     ffi.libc_srand(31)
     vo_mine = vo_frontend.VisualOdometry(win["fx"], win["fy"], win["cx"], win["cy"], winsize=4, user_config=user,
                                          solver=my_solver)
@@ -246,7 +255,7 @@ def test_vo_sequence_chained_windows_bit_exact():
         _compare(f"vo sequence window {k}", a, b)
     assert len(T_ref) == len(T_mine) == F + 1
     for a, b in zip(T_mine, T_ref):
-        assert np.array_equal(a, b)
+        assert ffi.bits_equal(a, b)
     # and the trajectory is the ground truth up to the monocular scale (loose: the point of this test is parity)
     gt = np.stack([np.concatenate([vo_frontend.matrix_to_rvec(win["Rs"][i]), win["ts"][i]]) for i in range(F)])
     T_gt = vo_frontend.formats.accumulate_poses(gt)
@@ -287,8 +296,8 @@ def test_mono_window_flag_variants_bit_exact(flags):
     args = (win["flows"], win["fx"], win["fy"], win["cx"], win["cy"])
     libc = __import__("ctypes").CDLL(None)
     ffi.libc_srand(90)
-    ref = oracle_host.run_window("ref", *args, config=cfg, boot=boot)
-    next_ref = libc.rand()
+    ref, next_ref = refgold.reference(lambda: (oracle_host.run_window("ref", *args, config=cfg, boot=boot),
+                                               libc.rand()))
     voldor_b200.set_bootstrap_override(*boot)
     ffi.libc_srand(90)
     mine = voldor_b200.voldor_ex(*args, config=cfg)
@@ -312,7 +321,7 @@ def test_mono_window_with_nonfinite_flow_pixels_bit_exact():
     cfg = f"--silent --max_iters {iters} --no_trunc_iters 1000 --n_poses_to_sample 1536"
     args = (flows, win["fx"], win["fy"], win["cx"], win["cy"])
     ffi.libc_srand(91)
-    ref = oracle_host.run_window("ref", *args, config=cfg, boot=boot)
+    ref = refgold.reference(lambda: oracle_host.run_window("ref", *args, config=cfg, boot=boot))
     voldor_b200.set_bootstrap_override(*boot)
     ffi.libc_srand(91)
     mine = voldor_b200.voldor_ex(*args, config=cfg)
@@ -338,7 +347,8 @@ def test_reference_cython_module_over_this_library_bit_exact():
     win, boot, _ = _mono_case(w, h, N, iters, seed=81)
     cfg = f"--silent --max_iters {iters} --no_trunc_iters 1000 --n_poses_to_sample 2048"
     ffi.libc_srand(92)
-    ref = oracle_host.run_window("ref", win["flows"], win["fx"], win["fy"], win["cx"], win["cy"], config=cfg, boot=boot)
+    ref = refgold.reference(lambda: oracle_host.run_window("ref", win["flows"], win["fx"], win["fy"], win["cx"],
+                                                           win["cy"], config=cfg, boot=boot))
     voldor_b200.set_bootstrap_override(*boot)
     ffi.libc_srand(92)
     py_voldor_kwargs = {"flows": win["flows"], "fx": float(win["fx"]), "fy": float(win["fy"]), "cx": float(win["cx"]),
@@ -348,4 +358,4 @@ def test_reference_cython_module_over_this_library_bit_exact():
     voldor_b200.set_bootstrap_override()
     assert mine["n_registered"] == ref["n_registered"] == N
     for k in ("poses", "poses_covar", "depth", "depth_conf"):
-        assert ffi.bits_equal(np.asarray(mine[k]), np.asarray(ref[k])), k
+        assert ffi.bits_equal(np.asarray(mine[k]), ref[k]), k
