@@ -85,6 +85,58 @@ def test_optimize_depth_variants(libs):
             assert rep_r["bit_mismatch"] == 0, rep_r
 
 
+def _route_sequence(lib, route):
+    """depth steps whose likelihood-term counts pick the different launch shapes of the search and the propagation"""
+    if route == "no_terms":
+        # a step with neither flows nor priors (every cost INF: the depth must stay, the random streams advance),
+        # then a two-flow step continuing on the same streams and the cached depth
+        win = synth.make_window(56, 40, 2, seed=21)
+        rc, d0, _, _ = lib.optimize_depth(56, 40, 0, depth=synth.noisy_depth(win), K=win["K"])
+        assert rc == 0
+        Rs, ts = synth.perturbed_poses(win)
+        rc, d1, r1, _ = lib.optimize_depth(56, 40, 2, flows=list(win["flows"]), rig=list(np.ones((2, 40, 56))),
+                                           Rs=list(Rs), ts=list(ts))
+        assert rc == 0
+        return d0, d1, r1
+    if route in ("one_flow", "eight_flows_gstep1"):
+        N, kw = (1, {}) if route == "one_flow" else (8, dict(gstep=1))
+        win = synth.make_window(68, 44, N, seed=22 + N)
+        Rs, ts = synth.perturbed_poses(win)
+        return [x for dr in _depth_sequence(lib, win, synth.noisy_depth(win), Rs, ts, n_calls=2, **kw) for x in dr]
+    assert route == "sixteen_flows_sixteen_priors"
+    w, h, N = 36, 28, 16
+    win = synth.make_window(w, h, N, seed=23)
+    Rs, ts = synth.perturbed_poses(win)
+    priors = [synth.noisy_depth(win, 0.02, seed=30 + p) for p in range(N)]
+    for p, prior in enumerate(priors):
+        prior[p:p + 3, 2 * p:2 * p + 5] = 0
+    pconfs = [np.full((h, w), 0.5 + 0.03 * p, np.float32) for p in range(N)]
+    confs = [np.ones((h, w), np.float32)] * N
+    dp_Rs, dp_ts = synth.perturbed_poses(win, 0.001, 0.01, seed=31)
+    kw = dict(basefocal=50.0, disp_delta=1.0)
+    rc, d1, r1, c1 = lib.optimize_depth(w, h, N, N, flows=list(win["flows"]), rig=list(np.ones((N, h, w), np.float32)),
+                                        depth=synth.noisy_depth(win), K=win["K"], Rs=list(Rs), ts=list(ts),
+                                        priors=priors, pconfs=pconfs, confs=confs, dp_Rs=list(dp_Rs),
+                                        dp_ts=list(dp_ts), **kw)
+    assert rc == 0
+    rc, d2, r2, c2 = lib.optimize_depth(w, h, N, N, Rs=list(Rs), ts=list(ts), **kw)
+    assert rc == 0
+    return d1, r1, c1, d2, r2, c2
+
+
+@pytest.mark.parametrize("route", ["no_terms", "one_flow", "eight_flows_gstep1", "sixteen_flows_sixteen_priors"])
+def test_optimize_depth_term_counts(libs, route):
+    """no likelihood term at all, one, eight with step-1 global propagation, and the most a step takes (16 + 16)"""
+    mine, ref = libs
+    a = _route_sequence(mine, route)
+    b = refgold.reference(lambda: _route_sequence(ref, route))
+    assert len(a) == len(b)
+    for k, (x, y) in enumerate(zip(a, b)):
+        rep = ffi.mismatch_report(x, y, f"optimize_depth {route} out{k}")
+        _report(rep)
+        assert rep["bit_mismatch"] == 0, rep
+
+
 def test_optimize_depth_with_priors(libs):
     mine, ref = libs
     w, h, N = 96, 64, 3

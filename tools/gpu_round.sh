@@ -68,12 +68,6 @@ PY
   done; done; done ;;
 weights)
   tools/_build/tex_probe weights $out/tex_weights.bin > $out/tex_weights.json 2>&1; cat $out/tex_weights.json ;;
-tpl)
-  # local propagation: two likelihood terms per lane instead of one, several windows in flight
-  for t in 1 2; do
-    VB_LOCAL_TPL=$t python bench.py --steps 6 --warmup 3 --inflight 6 --no-extras --no-cpu-baseline --no-parity > $out/bench_tpl$t.json 2> $out/bench_tpl$t.err
-    python -c "import json;l=json.loads(open('$out/bench_tpl$t.json').read().strip().splitlines()[-1]);print('TPL $t inflight 6 value',round(l['value'],1),'single',round(l['latency']['single_window']['value'],1), 'search ms', round(l['roofline']['avg_launch_ms'],4))" || tail -5 $out/bench_tpl$t.err
-  done ;;
 profile)
   # (1) top kernels, full sections, one launch each (one window of the benchmarked shape); raw + source pages are
   #     exported on the box, only the search-kernel report itself travels back (gpurun_out/ is capped at 64 MiB)
@@ -105,12 +99,6 @@ gpus2)
 gpus8)
   python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29518 bench.py --gpus 8 --steps 4 --warmup 3 --no-extras --no-cpu-baseline > $out/bench_gpus8.json 2> $out/bench_gpus8.err
   tail -c 1500 $out/bench_gpus8.json; tail -3 $out/bench_gpus8.err ;;
-prune)
-  for v in on off; do
-    if [ $v = off ]; then export VB_NO_SEARCH_PRUNING=1; else unset VB_NO_SEARCH_PRUNING; fi
-    python bench.py --steps 6 --warmup 3 --no-extras --no-cpu-baseline > $out/bench_prune_$v.json 2> $out/bench_prune_$v.err
-    python -c "import json;l=json.loads(open('$out/bench_prune_$v.json').read().strip().splitlines()[-1]);print('pruning $v: value',round(l['value'],1),'e2e',round(l['e2e']['value'],1),'single',round(l['latency']['single_window']['value'],1),'search ms',round(l['roofline']['avg_launch_ms'],4),'parity',l['parity_checked'])" || tail -5 $out/bench_prune_$v.err
-  done; unset VB_NO_SEARCH_PRUNING ;;
 probe)
   tools/_build/tex_probe 27 > $out/tex_probe.json 2>&1; cat $out/tex_probe.json ;;
 launches)

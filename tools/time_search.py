@@ -21,5 +21,5 @@ lib.vb_profile_enable(1)
 r = voldor_b200.voldor_ex(*args, config=cfg)
 ms, n = C.c_double(0), C.c_longlong(0)
 lib.vb_profile_get(C.byref(ms), C.byref(n))
-print("VB_SEARCH_BLOCK_Y", os.environ.get("VB_SEARCH_BLOCK_Y", "8"), "search ms/launch", ms.value / n.value, "launches", n.value,
+print("search ms/launch", ms.value / n.value, "launches", n.value,
       "window ms", r["stats_ms"][0])

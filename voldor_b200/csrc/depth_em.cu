@@ -14,7 +14,6 @@
 // Candidate costs use explicitly rounded FP32 arithmetic in the reference's evaluation order
 // (residual_model.cuh) because the argmin over candidates must reproduce the reference's decisions.
 #include "depth_em.cuh"
-#include <cstdlib>
 #include "residual_model.cuh"
 #include "geometry.cuh"
 #include <cmath>
@@ -44,73 +43,93 @@ struct DepthView {
 };
 
 // ------------------------------------------------------------------------------------------------
-// cost of hypothesising `depth` at pixel (px,py)   (reference: optimize_depth.cu:140-198)
+// The likelihood terms of hypothesising `depth` at a pixel (reference: optimize_depth.cu:84-138,140-198).
+// Every kernel that evaluates a term goes through these helpers, so the rounding order is written down once.
 // ------------------------------------------------------------------------------------------------
-// Frame 0 is always fetched at the pixel centre itself, so its observed flow, Fisk shape/scale and outlier density do
-// not depend on the candidate: callers that test several candidates per pixel pass them in (PRE0).
-struct Frame0Model {
-    float2 obs;
-    ObservedFlowModel m;
-};
-template <bool PRE0>
-__device__ __forceinline__ float pixel_cost_t(const DepthView& A, const CamBlock& C, const PriorCamBlock& PC, int px,
-                                              int py, float depth, const Frame0Model* f0) {
-    float cost_sum = 0.f;
-    float weight_sum = 0.f;
-    const float fpx = (float)px, fpy = (float)py;
-    const float fw = (float)A.w, fh = (float)A.h;
-
-    float ox, oy, oz;
-    backproject(C, fpx, fpy, depth, ox, oy, oz);
-    float px1 = fpx, py1 = fpy;
-    const float* wgt_ptr = A.rig + (size_t)py * A.pitch + px;
-
-    for (int f = 0; f < A.N; f++) {
-        float px2, py2;
-        rigid_move(C.R[f], C.t[f], ox, oy, oz);
-        project(C, ox, oy, oz, px2, py2);
-        if (oz > 0 && px1 >= 0 && px1 < fw && py1 >= 0 && py1 < fh) {
-            const float rfx = f_sub(px2, px1), rfy = f_sub(py2, py1);
-            float r;
-            if (PRE0 && f == 0) {
-                r = flow_rigidness_given(rfx, rfy, f0->obs.x, f0->obs.y, f0->m, A.abs_rf);
-            } else {
-                const float2 obs = fetch_stack<float2>(A.flows_tex, px1, py1, f, A.h);
-                r = flow_rigidness(rfx, rfy, obs.x, obs.y, A.lambda, A.abs_rf);
-            }
-            px1 = px2, py1 = py2;  // stale when the branch is not taken (SURVEY §9 Q6)
-            const float wgt = wgt_ptr[(size_t)f * A.plane];
-            cost_sum = f_fma(-wgt, logf(r), cost_sum);
-            weight_sum = f_add(weight_sum, wgt);
-        }
-    }
-
-    for (int f = 0; f < A.N_dp; f++) {
-        backproject(C, fpx, fpy, depth, ox, oy, oz);
-        rigid_move(PC.R[f], PC.t[f], ox, oy, oz);
-        project(C, ox, oy, oz, px1, py1);
-        if (oz > 0 && px1 >= 0 && px1 < fw && py1 >= 0 && py1 < fh) {
-            const float target_depth = fetch_stack<float>(A.dp_tex, px1, py1, f, A.h);
-            const float target_pconf = fetch_stack<float>(A.dp_pconf_tex, px1, py1, f, A.h);
-            const float target_conf = fetch_stack<float>(A.dp_conf_tex, px1, py1, f, A.h);
-            if (target_depth > 0) {
-                // prior 0 is the disparity prior when the caller passes disp_delta > 0 (SURVEY §9 Q21)
-                const float scale = (A.disp_delta > 0 && f == 0) ? A.disp_delta : A.delta;
-                const float wgt = f_mul(f_mul(target_pconf, target_conf), scale);
-                const float r = depth_rigidness(oz, target_depth, A.basefocal, A.omega, A.abs_rf);
-                cost_sum = f_fma(-wgt, logf(r), cost_sum);
-                weight_sum = f_add(weight_sum, wgt);
-            }
-        }
-    }
-
-    if (weight_sum == 0) return INFINITY;
-    return f_div(cost_sum, fmaxf(weight_sum, FLT_EPSILON));
+__device__ __forceinline__ bool in_image(const DepthView& A, float x, float y) {
+    return x >= 0 && x < (float)A.w && y >= 0 && y < (float)A.h;
 }
 
+// The chain of flow frames: the candidate's point is moved from frame to frame, and frame f fetches its observed flow
+// where the last frame that took part projected the point (the pixel itself before any did).
+struct FlowChain {
+    float ox, oy, oz;  // the point in the camera of the last frame stepped to
+    float px1, py1;    // fetch position of the next frame
+};
+__device__ __forceinline__ FlowChain flow_chain(const CamBlock& C, float fpx, float fpy, float depth) {
+    FlowChain ch;
+    backproject(C, fpx, fpy, depth, ch.ox, ch.oy, ch.oz);
+    ch.px1 = fpx, ch.py1 = fpy;
+    return ch;
+}
+// Steps the chain to frame f and projects the point to (px2, py2).  Frame f takes part when the point lies in front of
+// its camera and its fetch position (fx, fy) is inside the image; its rigid flow is then (px2 - fx, py2 - fy).  Only a
+// frame that takes part moves the fetch position on, so a later frame can fetch at a stale one (SURVEY §9 Q6).
+__device__ __forceinline__ bool flow_step(const DepthView& A, const CamBlock& C, int f, FlowChain& ch, float& fx,
+                                          float& fy, float& px2, float& py2) {
+    rigid_move(C.R[f], C.t[f], ch.ox, ch.oy, ch.oz);
+    project(C, ch.ox, ch.oy, ch.oz, px2, py2);
+    fx = ch.px1, fy = ch.py1;
+    if (!(ch.oz > 0 && in_image(A, fx, fy))) return false;
+    ch.px1 = px2, ch.py1 = py2;
+    return true;
+}
+
+// Depth prior p seen from the candidate: out of view when the point lies behind the prior's camera or projects outside
+// the image, no depth where the prior holds none, else the term takes part with weight `wgt` and posterior `r`.
+// Callers that need only one of the two leave the other to dead-code elimination.
+enum PriorSight { kPriorOutOfView, kPriorNoDepth, kPriorTakesPart };
+__device__ __forceinline__ PriorSight prior_term(const DepthView& A, const CamBlock& C, const PriorCamBlock& PC, int p,
+                                                 float fpx, float fpy, float depth, float& wgt, float& r) {
+    float ox, oy, oz, ux, uy;
+    backproject(C, fpx, fpy, depth, ox, oy, oz);
+    rigid_move(PC.R[p], PC.t[p], ox, oy, oz);
+    project(C, ox, oy, oz, ux, uy);
+    if (!(oz > 0 && in_image(A, ux, uy))) return kPriorOutOfView;
+    const float target_depth = fetch_stack<float>(A.dp_tex, ux, uy, p, A.h);
+    const float target_pconf = fetch_stack<float>(A.dp_pconf_tex, ux, uy, p, A.h);
+    const float target_conf = fetch_stack<float>(A.dp_conf_tex, ux, uy, p, A.h);
+    if (!(target_depth > 0)) return kPriorNoDepth;
+    // prior 0 is the disparity prior when the caller passes disp_delta > 0 (SURVEY §9 Q21)
+    const float scale = (A.disp_delta > 0 && p == 0) ? A.disp_delta : A.delta;
+    wgt = f_mul(f_mul(target_pconf, target_conf), scale);
+    r = depth_rigidness(oz, target_depth, A.basefocal, A.omega, A.abs_rf);
+    return kPriorTakesPart;
+}
+
+// The cost of a candidate: the weighted mean of -log r over the terms that take part, summed in term order
+// (flows f = 0..N-1, then priors 0..N_dp-1); INF when none does.
+struct CostSum {
+    float cost = 0.f, weight = 0.f;
+    __device__ __forceinline__ void add(float wgt, float log_r) {
+        cost = f_fma(-wgt, log_r, cost);
+        weight = f_add(weight, wgt);
+    }
+    __device__ __forceinline__ float value() const {
+        return weight == 0 ? INFINITY : f_div(cost, fmaxf(weight, FLT_EPSILON));
+    }
+};
+
+// cost of hypothesising `depth` at pixel (px,py)   (reference: optimize_depth.cu:140-198)
 __device__ float pixel_cost(const DepthView& A, const CamBlock& C, const PriorCamBlock& PC, int px, int py,
                             float depth) {
-    return pixel_cost_t<false>(A, C, PC, px, py, depth, nullptr);
+    const float fpx = (float)px, fpy = (float)py;
+    const float* wgt_ptr = A.rig + (size_t)py * A.pitch + px;
+    CostSum sum;
+    FlowChain ch = flow_chain(C, fpx, fpy, depth);
+    for (int f = 0; f < A.N; f++) {
+        float fx, fy, px2, py2;
+        if (flow_step(A, C, f, ch, fx, fy, px2, py2)) {
+            const float2 obs = fetch_stack<float2>(A.flows_tex, fx, fy, f, A.h);
+            const float r = flow_rigidness(f_sub(px2, fx), f_sub(py2, fy), obs.x, obs.y, A.lambda, A.abs_rf);
+            sum.add(wgt_ptr[(size_t)f * A.plane], logf(r));
+        }
+    }
+    for (int p = 0; p < A.N_dp; p++) {
+        float wgt, r;
+        if (prior_term(A, C, PC, p, fpx, fpy, depth, wgt, r) == kPriorTakesPart) sum.add(wgt, logf(r));
+    }
+    return sum.value();
 }
 
 __device__ __forceinline__ void try_candidate(const DepthView& A, const CamBlock& C, const PriorCamBlock& PC, int x,
@@ -159,61 +178,7 @@ __global__ void k_seed_rng(uint32_t* rng, int w, int h, int pitch, size_t plane)
 
 // ------------------------------------------------------------------------------------------------
 // fused: cost of the current depth + n_rand random candidates   (reference: optimize_depth.cu:269-284)
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256)
-    k_cost_and_random_search(const DepthView A, const __grid_constant__ CamBlock C,
-                             const __grid_constant__ PriorCamBlock PC, int n_rand) {
-    const int x = blockIdx.x * blockDim.x + threadIdx.x;
-    const int y = blockIdx.y * blockDim.y + threadIdx.y;
-    if (x >= A.w || y >= A.h) return;
-    const size_t idx = (size_t)y * A.pitch + x;
-
-    // it == -1 evaluates the current depth (the reference's compute_cost_map), it >= 0 the random draws
-    Xorwow s = {0, 0, 0, 0, 0, 0};
-    if (n_rand > 0) {
-        s.d = A.rng[idx];
-        s.v0 = A.rng[idx + A.plane];
-        s.v1 = A.rng[idx + 2 * A.plane];
-        s.v2 = A.rng[idx + 3 * A.plane];
-        s.v3 = A.rng[idx + 4 * A.plane];
-        s.v4 = A.rng[idx + 5 * A.plane];
-    }
-    float best_depth = A.depth[idx];
-    float best_cost = 0.f;
-    Frame0Model f0;
-    f0.obs = make_float2(0.f, 0.f);
-    f0.m.k.c = f0.m.k.s = f0.m.mu = 0.f;
-    if (A.N > 0) {
-        f0.obs = fetch_stack<float2>(A.flows_tex, (float)x, (float)y, 0, A.h);
-        f0.m = observed_flow_model(f0.obs.x, f0.obs.y, A.lambda, A.abs_rf);
-    }
-    for (int it = -1; it < n_rand; it++) {
-        float cand = best_depth;
-        if (it >= 0) {
-            const float u = xorwow_uniform(s);
-            // d = 1/(range_factor*U + 1/MAXIMUM_DEPTH)   (reference: optimize_depth.cu:273)
-            cand = __frcp_rn(f_fma(A.range_factor, u, 1.0f / kMaximumDepth));
-        }
-        const float c = pixel_cost_t<true>(A, C, PC, x, y, cand, &f0);
-        if (it < 0 || c < best_cost) {
-            best_depth = cand;
-            best_cost = c;
-        }
-    }
-    if (n_rand > 0) {
-        A.rng[idx] = s.d;
-        A.rng[idx + A.plane] = s.v0;
-        A.rng[idx + 2 * A.plane] = s.v1;
-        A.rng[idx + 3 * A.plane] = s.v2;
-        A.rng[idx + 4 * A.plane] = s.v3;
-        A.rng[idx + 5 * A.plane] = s.v4;
-    }
-    A.depth[idx] = best_depth;
-    A.cost[idx] = best_cost;
-}
-
-// ------------------------------------------------------------------------------------------------
-// The same search with EXACT early rejection of hopeless candidates, as a per-lane state machine.
+// with EXACT early rejection of hopeless candidates, as a per-lane state machine.
 //
 // A candidate is kept only if its cost S/W is strictly below the pixel's best cost.  Every likelihood term
 // -w*log(r) is >= 0 (w >= 0, r in [0,1]) and the weights are known before the candidate is evaluated, so after any
@@ -221,9 +186,10 @@ __global__ void __launch_bounds__(256)
 // candidate could collect.  Floating-point addition, fma with a non-negative product and division are monotone, so
 // the bound also holds for the rounded quantities: once  S_k >= round_up(best * max(W_ub, eps))  the reference's own
 // comparison `cost < best` is certain to fail and the remaining terms need not be evaluated.  No decision changes
-// (bit-identical depth / cost / RNG state: the parity tests run through this kernel); a pixel with a negative or NaN
-// weight, a NaN best cost or the evaluation of the current depth itself are never pruned.  On the benchmark windows a
-// random candidate survives 2.1 of its 8 terms on average (68 % are rejected by the first one).
+// (bit-identical depth / cost / RNG state); a pixel with a negative or NaN weight, a NaN best cost or the evaluation of
+// the current depth itself are never pruned.  On the benchmark windows a random candidate survives 2.1 of its 8 terms
+// on average (68 % are rejected by the first one).  Without any term every cost is INF: the current depth stays, no
+// draw is accepted (INF < INF fails, and reject_at is INF) and the stream still advances n_rand draws.
 //
 // Lanes would leave candidates at different frames, so each lane runs its own (candidate, frame) state machine and
 // every pass of the loop evaluates ONE term per lane: a lane that rejects early moves straight on to its next
@@ -248,7 +214,7 @@ __global__ void __launch_bounds__(256)
     const int y = blockIdx.y * blockDim.y + threadIdx.y;
     if (x >= A.w || y >= A.h) return;
     const size_t idx = (size_t)y * A.pitch + x;
-    const float fpx = (float)x, fpy = (float)y, fw = (float)A.w, fh = (float)A.h;
+    const float fpx = (float)x, fpy = (float)y;
 
     Xorwow s = {0, 0, 0, 0, 0, 0};
     if (n_rand > 0) {
@@ -261,12 +227,13 @@ __global__ void __launch_bounds__(256)
     }
     float best_depth = A.depth[idx];
     float best_cost = 0.f;
-    Frame0Model f0;
-    f0.obs = make_float2(0.f, 0.f);
-    f0.m.k.c = f0.m.k.s = f0.m.mu = 0.f;
+    // frame 0 always fetches at the pixel itself: its observed flow and Fisk model are the same for every candidate
+    float2 obs0 = make_float2(0.f, 0.f);
+    ObservedFlowModel m0;
+    m0.k.c = m0.k.s = m0.mu = 0.f;
     if (A.N > 0) {
-        f0.obs = fetch_stack<float2>(A.flows_tex, fpx, fpy, 0, A.h);
-        f0.m = observed_flow_model(f0.obs.x, f0.obs.y, A.lambda, A.abs_rf);
+        obs0 = fetch_stack<float2>(A.flows_tex, fpx, fpy, 0, A.h);
+        m0 = observed_flow_model(obs0.x, obs0.y, A.lambda, A.abs_rf);
     }
     // everything the flow terms of ANY candidate of this pixel can add to the weight sum, summed in term order
     const float* wgt_ptr = A.rig + idx;
@@ -280,83 +247,54 @@ __global__ void __launch_bounds__(256)
     const int n_terms = A.N + A.N_dp;
 
     int it = -1, f = 0;
-    float cand = best_depth, ox = 0.f, oy = 0.f, oz = 0.f, px1 = fpx, py1 = fpy;
-    float cost_sum = 0.f, weight_sum = 0.f, reject_at = 0.f;
+    float cand = best_depth, reject_at = 0.f;
+    FlowChain ch = {0.f, 0.f, 0.f, fpx, fpy};
+    CostSum sum;
     bool prune = false;
     while (true) {
         if (f == 0) {  // a new candidate: it == -1 is the current depth (never pruned), it >= 0 the random draws
             cand = best_depth;
             if (it >= 0) {
                 const float u = xorwow_uniform(s);
+                // d = 1/(range_factor*U + 1/MAXIMUM_DEPTH)   (reference: optimize_depth.cu:273)
                 cand = __frcp_rn(f_fma(A.range_factor, u, 1.0f / kMaximumDepth));
             }
-            backproject(C, fpx, fpy, cand, ox, oy, oz);
-            px1 = fpx, py1 = fpy;
-            cost_sum = 0.f, weight_sum = 0.f;
+            ch = flow_chain(C, fpx, fpy, cand);
+            sum = CostSum();
             prune = it >= 0 && weights_ok;
             if (prune) {
                 float w_ub = w_flows;
                 for (int p = 0; p < A.N_dp; p++) {  // the prior terms' weights depend on the candidate: look ahead
-                    float qx, qy, qz, ux, uy;
-                    backproject(C, fpx, fpy, cand, qx, qy, qz);
-                    rigid_move(PC.R[p], PC.t[p], qx, qy, qz);
-                    project(C, qx, qy, qz, ux, uy);
-                    if (qz > 0 && ux >= 0 && ux < fw && uy >= 0 && uy < fh) {
-                        const float target_depth = fetch_stack<float>(A.dp_tex, ux, uy, p, A.h);
-                        if (target_depth > 0) {
-                            const float scale = (A.disp_delta > 0 && p == 0) ? A.disp_delta : A.delta;
-                            const float wgt = f_mul(f_mul(fetch_stack<float>(A.dp_pconf_tex, ux, uy, p, A.h),
-                                                          fetch_stack<float>(A.dp_conf_tex, ux, uy, p, A.h)), scale);
-                            w_ub = f_add(w_ub, wgt);
-                            prune = prune && (wgt >= 0.f);
-                        }
+                    float wgt, r;
+                    if (prior_term(A, C, PC, p, fpx, fpy, cand, wgt, r) == kPriorTakesPart) {
+                        w_ub = f_add(w_ub, wgt);
+                        prune = prune && (wgt >= 0.f);
                     }
                 }
                 reject_at = __fmul_ru(best_cost, fmaxf(w_ub, FLT_EPSILON));
             }
         }
-        if (f < A.N) {  // likelihood term of flow f (pixel_cost_t, one pass of its loop)
-            float px2, py2;
-            rigid_move(C.R[f], C.t[f], ox, oy, oz);
-            project(C, ox, oy, oz, px2, py2);
-            if (oz > 0 && px1 >= 0 && px1 < fw && py1 >= 0 && py1 < fh) {
-                const float rfx = f_sub(px2, px1), rfy = f_sub(py2, py1);
-                float2 obs = f0.obs;
-                ObservedFlowModel m = f0.m;
+        if (f < A.N) {  // likelihood term of flow f
+            float fx, fy, px2, py2;
+            if (flow_step(A, C, f, ch, fx, fy, px2, py2)) {
+                float2 obs = obs0;
+                ObservedFlowModel m = m0;
                 if (f != 0) {
-                    obs = fetch_stack<float2>(A.flows_tex, px1, py1, f, A.h);
+                    obs = fetch_stack<float2>(A.flows_tex, fx, fy, f, A.h);
                     m = observed_flow_model(obs.x, obs.y, A.lambda, A.abs_rf);
                 }
-                const float r = flow_rigidness_given(rfx, rfy, obs.x, obs.y, m, A.abs_rf);
-                px1 = px2, py1 = py2;  // stale when the branch is not taken (SURVEY §9 Q6)
-                const float wgt = wgt_ptr[(size_t)f * A.plane];
-                cost_sum = f_fma(-wgt, logf(r), cost_sum);
-                weight_sum = f_add(weight_sum, wgt);
+                const float r = flow_rigidness_given(f_sub(px2, fx), f_sub(py2, fy), obs.x, obs.y, m, A.abs_rf);
+                sum.add(wgt_ptr[(size_t)f * A.plane], logf(r));
             }
         } else if (f < n_terms) {  // likelihood term of prior f - N
-            const int p = f - A.N;
-            float qx, qy, qz, ux, uy;
-            backproject(C, fpx, fpy, cand, qx, qy, qz);
-            rigid_move(PC.R[p], PC.t[p], qx, qy, qz);
-            project(C, qx, qy, qz, ux, uy);
-            if (qz > 0 && ux >= 0 && ux < fw && uy >= 0 && uy < fh) {
-                const float target_depth = fetch_stack<float>(A.dp_tex, ux, uy, p, A.h);
-                const float target_pconf = fetch_stack<float>(A.dp_pconf_tex, ux, uy, p, A.h);
-                const float target_conf = fetch_stack<float>(A.dp_conf_tex, ux, uy, p, A.h);
-                if (target_depth > 0) {
-                    const float scale = (A.disp_delta > 0 && p == 0) ? A.disp_delta : A.delta;
-                    const float wgt = f_mul(f_mul(target_pconf, target_conf), scale);
-                    const float r = depth_rigidness(qz, target_depth, A.basefocal, A.omega, A.abs_rf);
-                    cost_sum = f_fma(-wgt, logf(r), cost_sum);
-                    weight_sum = f_add(weight_sum, wgt);
-                }
-            }
+            float wgt, r;
+            if (prior_term(A, C, PC, f - A.N, fpx, fpy, cand, wgt, r) == kPriorTakesPart) sum.add(wgt, logf(r));
         }
         f++;
-        const bool rejected = prune && cost_sum >= reject_at;
+        const bool rejected = prune && sum.cost >= reject_at;
         if (f >= n_terms || rejected) {
             if (!rejected) {
-                const float c = weight_sum == 0 ? INFINITY : f_div(cost_sum, fmaxf(weight_sum, FLT_EPSILON));
+                const float c = sum.value();
                 if (it < 0 || c < best_cost) best_depth = cand, best_cost = c;
             }
             it++, f = 0;
@@ -382,7 +320,6 @@ __global__ void __launch_bounds__(256)
 // (reference: optimize_depth.cu:209-235)
 // ------------------------------------------------------------------------------------------------
 enum { DIR_L2R = 0, DIR_T2B = 1, DIR_R2L = 2, DIR_B2T = 3 };
-constexpr int kLocalTermsPerLane = 1;  // default split of a candidate's likelihood terms over lanes
 
 template <int DIR>
 __global__ void __launch_bounds__(128)
@@ -405,90 +342,46 @@ __global__ void __launch_bounds__(128)
 }
 
 // ------------------------------------------------------------------------------------------------
-// local propagation: sequential chain inside each `width`-pixel segment (reference: optimize_depth.cu:237-267)
-// thread (seg, o): seg = segment index along the propagation axis, o = index along the other axis.
-// Also serves global propagation with step == 1 (one segment = the whole row/column).
-// ------------------------------------------------------------------------------------------------
-template <int DIR>
-__global__ void __launch_bounds__(128)
-    k_local_propagation(const DepthView A, const __grid_constant__ CamBlock C,
-                        const __grid_constant__ PriorCamBlock PC, int width) {
-    const int o = blockIdx.x * blockDim.x + threadIdx.x;
-    const int seg = blockIdx.y * blockDim.y + threadIdx.y;
-    if (DIR == DIR_L2R) {
-        if (o >= A.h) return;
-        const int p0 = seg * width;
-        if (p0 >= A.w) return;
-        const int lo = max(1, p0 + 1), hi = min(A.w, p0 + width);
-        for (int x = lo; x < hi; x++) try_candidate(A, C, PC, x, o, A.depth[(size_t)o * A.pitch + x - 1]);
-    } else if (DIR == DIR_R2L) {
-        if (o >= A.h) return;
-        const int p0 = seg * width;
-        if (p0 >= A.w) return;
-        for (int x = min(A.w - 2, p0 + width - 2); x >= max(0, p0); x--)
-            try_candidate(A, C, PC, x, o, A.depth[(size_t)o * A.pitch + x + 1]);
-    } else if (DIR == DIR_T2B) {
-        if (o >= A.w) return;
-        const int p0 = seg * width;
-        if (p0 >= A.h) return;
-        const int lo = max(1, p0 + 1), hi = min(A.h, p0 + width);
-        for (int y = lo; y < hi; y++) try_candidate(A, C, PC, o, y, A.depth[(size_t)(y - 1) * A.pitch + o]);
-    } else {
-        if (o >= A.w) return;
-        const int p0 = seg * width;
-        if (p0 >= A.h) return;
-        for (int y = min(A.h - 2, p0 + width - 2); y >= max(0, p0); y--)
-            try_candidate(A, C, PC, o, y, A.depth[(size_t)(y + 1) * A.pitch + o]);
-    }
-}
-
-// ------------------------------------------------------------------------------------------------
 // Cooperative candidate cost: the N flow terms and N_dp prior terms of ONE candidate are evaluated by a group
-// of G lanes (one term per lane: the texture fetch and the ~600-instruction Fisk posterior run in parallel),
-// then combined in the reference's order f = 0..N-1, priors 0..N_dp-1 with the same fused multiply-adds, so
+// of G >= N + N_dp lanes (one term per lane: the texture fetch and the ~600-instruction Fisk posterior run in
+// parallel), then combined in the reference's order f = 0..N-1, priors 0..N_dp-1 with the same fused multiply-adds, so
 // the result is bit-identical to pixel_cost().  The fetch position of frame f depends on the in-view tests of all
 // earlier frames (stale px1 rule, SURVEY §9 Q6): either every lane walks the whole pose chain for itself (SHARE =
 // false, shortest dependent path — small launches), or the lanes share the projections and settle the rule with two
 // ballots (SHARE = true, a fifth fewer instructions — launches that fill the GPU; see launch_local_group).
 // The result is returned on every lane of the group.
 // ------------------------------------------------------------------------------------------------
-template <int G, int TPL, bool SHARE>
+template <int G, bool SHARE>
 __device__ __forceinline__ float pixel_cost_group(const DepthView& A, const CamBlock& C, const PriorCamBlock& PC,
                                                   int px, int py, float depth, int gl, unsigned gmask, int gbase) {
-    // lane gl owns the terms k = gl, gl+G, ... (slot k/G); terms 0..N-1 are flows, N..N+N_dp-1 priors
+    // lane gl owns term gl: terms 0..N-1 are flows, N..N+N_dp-1 priors
     const float fpx = (float)px, fpy = (float)py;
-    const float fw = (float)A.w, fh = (float)A.h;
-    float ox, oy, oz;
-    backproject(C, fpx, fpy, depth, ox, oy, oz);
-    float px1 = fpx, py1 = fpy;
-    float m_px1[TPL], m_py1[TPL], m_px2[TPL], m_py2[TPL];
-    bool my_valid[TPL];
-    float my_w[TPL], my_log[TPL];
-#pragma unroll
-    for (int j = 0; j < TPL; j++) my_valid[j] = false, my_w[j] = 0.f, my_log[j] = 0.f, m_px1[j] = m_py1[j] = m_px2[j] = m_py2[j] = 0.f;
-    if constexpr (TPL == 1 && SHARE) {
-        // One term per lane: every lane still walks the rigid moves (frame f's camera-space point is a running
-        // product), but only lane f projects frame f — the two IEEE divisions and the in-view tests of a frame are
-        // done once per group instead of once per lane.  Which frames take part and where each one fetches from
-        // (the position of the last earlier frame that took part, or the pixel itself) follows from two group-wide
-        // bit masks: Z_f = "point in front of camera f", P_f = "projection of frame f inside the image".
-        float mx = 0.f, my = 0.f, mz = 0.f;
+    float fx = 0.f, fy = 0.f, px2 = 0.f, py2 = 0.f;
+    bool valid = false;
+    float my_w = 0.f, my_log = 0.f;
+    if constexpr (SHARE) {
+        // Every lane still walks the rigid moves (frame f's camera-space point is a running product), but only lane f
+        // projects frame f — the two IEEE divisions and the in-view tests of a frame are done once per group instead
+        // of once per lane.  Which frames take part and where each one fetches from (the position of the last earlier
+        // frame that took part, or the pixel itself) follows from two group-wide bit masks: Z_f = "point in front of
+        // camera f", P_f = "projection of frame f inside the image".
+        float ox, oy, oz, mx = 0.f, my = 0.f, mz = 0.f;
+        backproject(C, fpx, fpy, depth, ox, oy, oz);
         for (int f = 0; f < A.N; f++) {
             rigid_move(C.R[f], C.t[f], ox, oy, oz);
             if (f == gl) mx = ox, my = oy, mz = oz;
         }
-        float px2 = 0.f, py2 = 0.f;
         bool in_front = false, inside = false;
         if (gl < A.N) {
             project(C, mx, my, mz, px2, py2);
             in_front = mz > 0;
-            inside = px2 >= 0 && px2 < fw && py2 >= 0 && py2 < fh;
+            inside = in_image(A, px2, py2);
         }
         const unsigned zb = __ballot_sync(gmask, in_front) >> gbase;
         const unsigned pb = __ballot_sync(gmask, inside) >> gbase;
         const unsigned all = (A.N >= 32) ? 0xffffffffu : ((1u << A.N) - 1u);
         int src = gl - 1;  // frame whose projected position this lane's frame fetches at; -1 = the pixel itself
-        bool valid = gl < A.N;
+        valid = gl < A.N;
         if ((zb & pb & all) != all) {
             // some frame drops out: replay the reference's sequential rule (stale px1, SURVEY §9 Q6) on the masks
             bool at_inside = true;  // the pixel itself lies inside the image
@@ -502,69 +395,42 @@ __device__ __forceinline__ float pixel_cost_group(const DepthView& A, const CamB
         }
         const float sx = __shfl_sync(gmask, px2, gbase + max(src, 0));
         const float sy = __shfl_sync(gmask, py2, gbase + max(src, 0));
-        m_px1[0] = src < 0 ? fpx : sx, m_py1[0] = src < 0 ? fpy : sy;
-        m_px2[0] = px2, m_py2[0] = py2, my_valid[0] = valid;
+        fx = src < 0 ? fpx : sx, fy = src < 0 ? fpy : sy;
     } else {
+        FlowChain ch = flow_chain(C, fpx, fpy, depth);
         for (int f = 0; f < A.N; f++) {
-            float px2, py2;
-            rigid_move(C.R[f], C.t[f], ox, oy, oz);
-            project(C, ox, oy, oz, px2, py2);
-            if (oz > 0 && px1 >= 0 && px1 < fw && py1 >= 0 && py1 < fh) {
-#pragma unroll
-                for (int j = 0; j < TPL; j++)
-                    if (f == gl + j * G) m_px1[j] = px1, m_py1[j] = py1, m_px2[j] = px2, m_py2[j] = py2, my_valid[j] = true;
-                px1 = px2, py1 = py2;
-            }
+            float sfx, sfy, spx2, spy2;
+            if (flow_step(A, C, f, ch, sfx, sfy, spx2, spy2) && f == gl)
+                fx = sfx, fy = sfy, px2 = spx2, py2 = spy2, valid = true;
         }
     }
-#pragma unroll
-    for (int j = 0; j < TPL; j++) {
-        const int k = gl + j * G;
-        if (my_valid[j]) {
-            const float2 obs = fetch_stack<float2>(A.flows_tex, m_px1[j], m_py1[j], k, A.h);
-            const float rfx = f_sub(m_px2[j], m_px1[j]), rfy = f_sub(m_py2[j], m_py1[j]);
-            my_w[j] = A.rig[(size_t)k * A.plane + (size_t)py * A.pitch + px];
-            my_log[j] = logf(flow_rigidness(rfx, rfy, obs.x, obs.y, A.lambda, A.abs_rf));
-        }
-        const int pf = k - A.N;
-        if (pf >= 0 && pf < A.N_dp) {
-            backproject(C, fpx, fpy, depth, ox, oy, oz);
-            rigid_move(PC.R[pf], PC.t[pf], ox, oy, oz);
-            project(C, ox, oy, oz, px1, py1);
-            if (oz > 0 && px1 >= 0 && px1 < fw && py1 >= 0 && py1 < fh) {
-                const float target_depth = fetch_stack<float>(A.dp_tex, px1, py1, pf, A.h);
-                const float target_pconf = fetch_stack<float>(A.dp_pconf_tex, px1, py1, pf, A.h);
-                const float target_conf = fetch_stack<float>(A.dp_conf_tex, px1, py1, pf, A.h);
-                if (target_depth > 0) {
-                    const float scale = (A.disp_delta > 0 && pf == 0) ? A.disp_delta : A.delta;
-                    my_w[j] = f_mul(f_mul(target_pconf, target_conf), scale);
-                    my_log[j] = logf(depth_rigidness(oz, target_depth, A.basefocal, A.omega, A.abs_rf));
-                    my_valid[j] = true;
-                }
-            }
-        }
+    if (valid) {
+        const float2 obs = fetch_stack<float2>(A.flows_tex, fx, fy, gl, A.h);
+        my_w = A.rig[(size_t)gl * A.plane + (size_t)py * A.pitch + px];
+        my_log = logf(flow_rigidness(f_sub(px2, fx), f_sub(py2, fy), obs.x, obs.y, A.lambda, A.abs_rf));
     }
-    float cost_sum = 0.f, weight_sum = 0.f;
-    const int terms = A.N + A.N_dp;
-#pragma unroll
-    for (int j = 0; j < TPL; j++) {
-        const unsigned taking_part = __ballot_sync(gmask, my_valid[j]) >> gbase;
-        for (int k = j * G; k < terms && k < (j + 1) * G; k++) {
-            const float w = __shfl_sync(gmask, my_w[j], gbase + k - j * G);
-            const float lg = __shfl_sync(gmask, my_log[j], gbase + k - j * G);
-            if ((taking_part >> (k - j * G)) & 1u) {
-                cost_sum = f_fma(-w, lg, cost_sum);
-                weight_sum = f_add(weight_sum, w);
-            }
-        }
+    const int pf = gl - A.N;
+    if (pf >= 0 && pf < A.N_dp) {
+        float wgt, r;
+        if (prior_term(A, C, PC, pf, fpx, fpy, depth, wgt, r) == kPriorTakesPart)
+            my_w = wgt, my_log = logf(r), valid = true;
     }
-    if (weight_sum == 0) return INFINITY;
-    return f_div(cost_sum, fmaxf(weight_sum, FLT_EPSILON));
+    CostSum sum;
+    const unsigned taking_part = __ballot_sync(gmask, valid) >> gbase;
+    for (int k = 0; k < A.N + A.N_dp && k < G; k++) {
+        const float w = __shfl_sync(gmask, my_w, gbase + k);
+        const float lg = __shfl_sync(gmask, my_log, gbase + k);
+        if ((taking_part >> k) & 1u) sum.add(w, lg);
+    }
+    return sum.value();
 }
 
-// local propagation with G lanes per chain: block = 128 threads = 128/G chains.
-// chain index c -> (o, seg) with o fastest.
-template <int DIR, int G, int TPL, bool SHARE>
+// ------------------------------------------------------------------------------------------------
+// local propagation: sequential chain inside each `width`-pixel segment (reference: optimize_depth.cu:237-267),
+// with G lanes per chain: block = 128 threads = 128/G chains.  chain index c -> (o, seg) with o fastest, o = index
+// along the other axis.  Also serves global propagation with step == 1 (one segment = the whole row/column).
+// ------------------------------------------------------------------------------------------------
+template <int DIR, int G, bool SHARE>
 __global__ void __launch_bounds__(128)
     k_local_propagation_group(const DepthView A, const __grid_constant__ CamBlock C,
                               const __grid_constant__ PriorCamBlock PC, int width, int n_other, int n_seg) {
@@ -604,7 +470,7 @@ __global__ void __launch_bounds__(128)
         if (i >= count) break;
         const int x = rowdir ? pos : o, y = rowdir ? o : pos;
         const size_t idx = (size_t)y * A.pitch + x;
-        const float c = pixel_cost_group<G, TPL, SHARE>(A, C, PC, x, y, cand, gl, gmask, gbase);
+        const float c = pixel_cost_group<G, SHARE>(A, C, PC, x, y, cand, gl, gmask, gbase);
         const float cur_cost = A.cost[idx];
         if (c < cur_cost) {
             if (gl == 0) A.depth[idx] = cand, A.cost[idx] = c;
@@ -628,38 +494,28 @@ __global__ void __launch_bounds__(256)
     if (x >= A.w || y >= A.h) return;
     const size_t idx = (size_t)y * A.pitch + x;
     const float fpx = (float)x, fpy = (float)y;
-    const float fw = (float)A.w, fh = (float)A.h;
     const float depth = A.depth[idx];
 
-    float ox, oy, oz;
-    backproject(C, fpx, fpy, depth, ox, oy, oz);
-    float px1 = fpx, py1 = fpy;
+    FlowChain ch = flow_chain(C, fpx, fpy, depth);
     for (int f = 0; f < A.N; f++) {
-        float px2, py2;
-        rigid_move(C.R[f], C.t[f], ox, oy, oz);
-        project(C, ox, oy, oz, px2, py2);
+        float fx, fy, px2, py2;
         float r = 0.f;
-        if (oz > 0 && px1 >= 0 && px1 < fw && py1 >= 0 && py1 < fh) {
-            const float2 obs = fetch_stack<float2>(A.flows_tex, px1, py1, f, A.h);
-            const float rfx = f_sub(px2, px1), rfy = f_sub(py2, py1);
-            px1 = px2, py1 = py2;
-            r = flow_rigidness(rfx, rfy, obs.x, obs.y, A.lambda, A.abs_rf);
+        if (flow_step(A, C, f, ch, fx, fy, px2, py2)) {
+            const float2 obs = fetch_stack<float2>(A.flows_tex, fx, fy, f, A.h);
+            r = flow_rigidness(f_sub(px2, fx), f_sub(py2, fy), obs.x, obs.y, A.lambda, A.abs_rf);
         }
         A.rig[idx + (size_t)f * A.plane] = r;
     }
 
-    for (int f = 0; f < A.N_dp; f++) {
-        backproject(C, fpx, fpy, depth, ox, oy, oz);
-        rigid_move(PC.R[f], PC.t[f], ox, oy, oz);
-        project(C, ox, oy, oz, px1, py1);
-        float* conf = A.dp_conf + (size_t)f * A.dp_conf_plane + (size_t)y * A.dp_conf_pitch + x;
-        if (oz > 0 && px1 >= 0 && px1 < fw && py1 >= 0 && py1 < fh) {
-            const float target_depth = fetch_stack<float>(A.dp_tex, px1, py1, f, A.h);
-            // confidence is left untouched where the prior has no depth (SURVEY §9 Q19)
-            if (target_depth > 0) *conf = depth_rigidness(oz, target_depth, A.basefocal, A.omega, A.abs_rf);
-        } else {
+    for (int p = 0; p < A.N_dp; p++) {
+        float* conf = A.dp_conf + (size_t)p * A.dp_conf_plane + (size_t)y * A.dp_conf_pitch + x;
+        float wgt, r;
+        const PriorSight sight = prior_term(A, C, PC, p, fpx, fpy, depth, wgt, r);
+        // confidence is left untouched where the prior has no depth (SURVEY §9 Q19)
+        if (sight == kPriorTakesPart)
+            *conf = r;
+        else if (sight == kPriorOutOfView)
             *conf = 0.f;
-        }
     }
 }
 
@@ -819,13 +675,59 @@ void fb_smooth_stack(StackView E_in, StackView E, StackView F, StackView B, int 
     k_fb_posterior<<<pg, pb, 0, s>>>(E, F, B, w, h);
 }
 
+// One lane per likelihood term of a candidate (see pixel_cost_group): a 31-long chain then costs ~1 term of latency per
+// step instead of N + N_dp.  G is the smallest power of two >= max(N + N_dp, 1), so one warp always holds a group.
+static_assert(kMaxFrames + kMaxPriorFrames <= 32, "the likelihood terms of a candidate must fit one warp");
+
+template <int DIR, int G>
+void launch_local_group(const DepthView& A, const CamBlock& C, const PriorCamBlock& PC, int width, int other,
+                        int nseg, cudaStream_t s) {
+    const long long threads = (long long)other * nseg * G;
+    const unsigned blocks = (unsigned)VB_DIV_CEIL(threads, 128);
+    // Sharing the projections of a candidate across the lanes of its group (pixel_cost_group) removes a fifth of the
+    // instructions but lengthens the dependent path of one evaluation (projection -> ballot -> shuffle -> fetch instead
+    // of projections overlapping the next rigid move).  Measured alone: 0.449 -> 0.401 ms at 16 warps per SM (640x480x8),
+    // 0.307 -> 0.375 ms at 2 warps per SM (320x240x4).  A launch that cannot fill the GPU anyway keeps every lane
+    // self-contained.
+    static const int sms = [] {
+        int dev = 0, n = 148;
+        cudaGetDevice(&dev);
+        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
+        return n;
+    }();
+    if (threads / 32 >= 8LL * sms)
+        k_local_propagation_group<DIR, G, true><<<blocks, 128, 0, s>>>(A, C, PC, width, other, nseg);
+    else
+        k_local_propagation_group<DIR, G, false><<<blocks, 128, 0, s>>>(A, C, PC, width, other, nseg);
+}
+
+template <int DIR>
+void launch_local(const DepthView& A, const CamBlock& C, const PriorCamBlock& PC, int width, cudaStream_t s) {
+    const bool rowdir = (DIR == DIR_L2R || DIR == DIR_R2L);
+    const int len = rowdir ? A.w : A.h, other = rowdir ? A.h : A.w;
+    const int nseg = VB_DIV_CEIL(len, width);
+    const int terms = A.N + A.N_dp;
+    if (terms > 16)
+        launch_local_group<DIR, 32>(A, C, PC, width, other, nseg, s);
+    else if (terms > 8)
+        launch_local_group<DIR, 16>(A, C, PC, width, other, nseg, s);
+    else if (terms > 4)
+        launch_local_group<DIR, 8>(A, C, PC, width, other, nseg, s);
+    else if (terms > 2)
+        launch_local_group<DIR, 4>(A, C, PC, width, other, nseg, s);
+    else if (terms > 1)
+        launch_local_group<DIR, 2>(A, C, PC, width, other, nseg, s);
+    else
+        launch_local_group<DIR, 1>(A, C, PC, width, other, nseg, s);
+}
+
 template <int DIR>
 void launch_global(const DepthView& A, const CamBlock& C, const PriorCamBlock& PC, int step, cudaStream_t s) {
     const bool rowdir = (DIR == DIR_L2R || DIR == DIR_R2L);
     const int len = rowdir ? A.w : A.h, other = rowdir ? A.h : A.w;
     if (step == 1) {
-        // a chain: identical to local propagation with one segment spanning the whole axis
-        k_local_propagation<DIR><<<dim3(VB_DIV_CEIL(other, 128), 1), dim3(128, 1), 0, s>>>(A, C, PC, len);
+        // a chain: local propagation with one segment spanning the whole axis
+        launch_local<DIR>(A, C, PC, len, s);
         return;
     }
     const int n = (len - 2) / step + 1;  // number of evaluated positions along the axis (len >= 2)
@@ -836,67 +738,22 @@ void launch_global(const DepthView& A, const CamBlock& C, const PriorCamBlock& P
         k_global_propagation<DIR><<<dim3(VB_DIV_CEIL(n, 4), VB_DIV_CEIL(other, 32)), dim3(4, 32), 0, s>>>(A, C, PC, step);
 }
 
-template <int DIR, int G, int TPL>
-void launch_local_group(const DepthView& A, const CamBlock& C, const PriorCamBlock& PC, int width, int other,
-                        int nseg, cudaStream_t s) {
-    const long long threads = (long long)other * nseg * G;
-    const unsigned blocks = (unsigned)VB_DIV_CEIL(threads, 128);
-    // Sharing the projections of a candidate across the lanes of its group (pixel_cost_group) removes a fifth of the
-    // instructions but lengthens the dependent path of one evaluation (projection -> ballot -> shuffle -> fetch instead
-    // of projections overlapping the next rigid move).  Measured alone: 0.449 -> 0.401 ms at 16 warps per SM (640x480x8),
-    // 0.307 -> 0.375 ms at 2 warps per SM (320x240x4).  A launch that cannot fill the GPU anyway keeps every lane
-    // self-contained.  VB_LOCAL_SHARE=0/1 forces one variant (profiling).
-    static const int forced = [] { const char* e = getenv("VB_LOCAL_SHARE"); return e ? atoi(e) : -1; }();
-    static const int sms = [] {
-        int dev = 0, n = 148;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-        return n;
-    }();
-    const bool share = TPL == 1 && (forced >= 0 ? forced != 0 : threads / 32 >= 8LL * sms);
-    if (share)
-        k_local_propagation_group<DIR, G, TPL, TPL == 1><<<blocks, 128, 0, s>>>(A, C, PC, width, other, nseg);
-    else
-        k_local_propagation_group<DIR, G, TPL, false><<<blocks, 128, 0, s>>>(A, C, PC, width, other, nseg);
-}
-
-template <int DIR>
-void launch_local(const DepthView& A, const CamBlock& C, const PriorCamBlock& PC, int width, cudaStream_t s) {
-    const bool rowdir = (DIR == DIR_L2R || DIR == DIR_R2L);
-    const int len = rowdir ? A.w : A.h, other = rowdir ? A.h : A.w;
-    const int nseg = VB_DIV_CEIL(len, width);
-    const int terms = A.N + A.N_dp;
-    // one lane per likelihood term of a candidate (see pixel_cost_group); a 31-long chain then costs ~1 term of
-    // latency per step instead of N
-    // lanes per chain G and terms per lane TPL (G * TPL >= terms).  One term per lane minimises the latency of a
-    // chain step; two terms per lane halve the warps and the redundant pose-chain walks — the better trade when
-    // the launch is issue bound.  VB_LOCAL_TPL overrides (profiling).
-    static const int forced_tpl = [] { const char* e = getenv("VB_LOCAL_TPL"); return e ? atoi(e) : 0; }();
-    const int tpl = forced_tpl > 0 ? forced_tpl : kLocalTermsPerLane;
-    const int lanes = VB_DIV_CEIL(terms, tpl);
-    const int G = lanes > 16 ? 32 : lanes > 8 ? 16 : lanes > 4 ? 8 : lanes > 2 ? 4 : lanes > 1 ? 2 : 1;
-#define VB_LOCAL_CASE(g)                                                              \
-    if (G == g) {                                                                     \
-        if (g >= terms)                                                               \
-            launch_local_group<DIR, g, 1>(A, C, PC, width, other, nseg, s);           \
-        else if (2 * g >= terms)                                                      \
-            launch_local_group<DIR, g, 2>(A, C, PC, width, other, nseg, s);           \
-        else                                                                          \
-            launch_local_group<DIR, g, 4>(A, C, PC, width, other, nseg, s);           \
-        return;                                                                       \
+// Adds the duration of what issue() enqueues on stream s to (ms, count) when profiling is switched on.  Timing a
+// region needs a sync, so it is only done then.
+template <class Issue>
+void timed(KernelProfile& prof, cudaStream_t s, double& ms, long long& count, Issue&& issue) {
+    if (!prof.enabled) {
+        issue();
+        return;
     }
-    if (terms >= 2 && 4 * G >= terms) {
-        VB_LOCAL_CASE(32)
-        VB_LOCAL_CASE(16)
-        VB_LOCAL_CASE(8)
-        VB_LOCAL_CASE(4)
-        VB_LOCAL_CASE(2)
-    }
-#undef VB_LOCAL_CASE
-    if (terms >= 2 && G == 1) {
-        // a whole candidate per lane is what the plain kernel does
-    }
-        k_local_propagation<DIR><<<dim3(VB_DIV_CEIL(other, 32), VB_DIV_CEIL(nseg, 4)), dim3(32, 4), 0, s>>>(A, C, PC, width);
+    if (!prof.ev0) cudaEventCreate(&prof.ev0), cudaEventCreate(&prof.ev1);
+    cudaEventRecord(prof.ev0, s);
+    issue();
+    cudaEventRecord(prof.ev1, s);
+    cudaEventSynchronize(prof.ev1);
+    float t = 0;
+    cudaEventElapsedTime(&t, prof.ev0, prof.ev1);
+    ms += t, count++;
 }
 
 }  // namespace
@@ -926,8 +783,6 @@ void DepthEM::invalidate_smoothing() {
 // Block height of the 1-thread-per-pixel search kernel: pick the shape whose grid fills the last wave best
 // (tail balance on 148 SMs); resident blocks per SM come from the occupancy calculator.
 static int pick_search_block_y(int w, int h, int n_sm) {
-    static const int forced = [] { const char* e = getenv("VB_SEARCH_BLOCK_Y"); return e ? atoi(e) : 0; }();
-    if (forced > 0 && forced <= 8) return forced;
     static int per_sm[9] = {0};
     static std::mutex per_sm_mutex;  // contexts call this from different host threads
     std::lock_guard<std::mutex> lock(per_sm_mutex);
@@ -937,7 +792,9 @@ static int pick_search_block_y(int w, int h, int n_sm) {
     for (int by : cand) {
         if (!per_sm[by]) {
             int nb = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_cost_and_random_search, 32 * by, 0) != cudaSuccess || nb < 1)
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_cost_and_random_search_pruned, 32 * by, 0) !=
+                    cudaSuccess ||
+                nb < 1)
                 nb = 1;
             per_sm[by] = nb;
         }
@@ -997,6 +854,8 @@ int DepthEM::run(int N, int N_dp, const DepthHyper& hp, bool update_rigidness_on
     A.dp_conf_pitch = (int)(dp_conf.pitch / sizeof(float));
     A.dp_conf_plane = (size_t)A.dp_conf_pitch * h;
 
+    KernelProfile none;  // counters of a context that does not profile
+    KernelProfile& prof = this->prof ? *this->prof : none;
     cudaStream_t s = stream;
     const dim3 pb(32, 8), pg(VB_DIV_CEIL(w, 32), VB_DIV_CEIL(h, 8));
 
@@ -1028,29 +887,11 @@ int DepthEM::run(int N, int N_dp, const DepthHyper& hp, bool update_rigidness_on
             }
             VB_RETURN_IF_CUDA_ERROR();
         }
-        KernelProfile none;
-        KernelProfile& prof = this->prof ? *this->prof : none;
-        if (prof.enabled) {
-            if (!prof.ev0) cudaEventCreate(&prof.ev0), cudaEventCreate(&prof.ev1);
-            cudaEventRecord(prof.ev0, s);
-        }
-        {
+        timed(prof, s, prof.search_ms, prof.search_launches, [&] {
             const int by = pick_search_block_y(w, h, n_sm);
             const dim3 sb(32, by), sg(VB_DIV_CEIL(w, 32), VB_DIV_CEIL(h, by));
-            static const bool no_pruning = getenv("VB_NO_SEARCH_PRUNING") != nullptr;  // A/B measurement
-            if (N + N_dp > 0 && !no_pruning)
-                k_cost_and_random_search_pruned<<<sg, sb, 0, s>>>(A, cam, pcam, hp.n_rand_samples);
-            else
-                k_cost_and_random_search<<<sg, sb, 0, s>>>(A, cam, pcam, hp.n_rand_samples);
-        }
-        if (prof.enabled) {
-            // timing one kernel needs a sync; only done when profiling is switched on
-            cudaEventRecord(prof.ev1, s);
-            cudaEventSynchronize(prof.ev1);
-            float ms = 0;
-            cudaEventElapsedTime(&ms, prof.ev0, prof.ev1);
-            prof.search_ms += ms, prof.search_launches++;
-        }
+            k_cost_and_random_search_pruned<<<sg, sb, 0, s>>>(A, cam, pcam, hp.n_rand_samples);
+        });
         VB_RETURN_IF_CUDA_ERROR();
         if (hp.global_prop_step > 0) {
             launch_global<DIR_L2R>(A, cam, pcam, hp.global_prop_step, s);
@@ -1059,38 +900,17 @@ int DepthEM::run(int N, int N_dp, const DepthHyper& hp, bool update_rigidness_on
             launch_global<DIR_T2B>(A, cam, pcam, hp.global_prop_step, s);
         }
         if (hp.local_prop_width > 0) {
-            if (prof.enabled) cudaEventRecord(prof.ev0, s);
-            launch_local<DIR_L2R>(A, cam, pcam, hp.local_prop_width, s);
-            launch_local<DIR_B2T>(A, cam, pcam, hp.local_prop_width, s);
-            launch_local<DIR_R2L>(A, cam, pcam, hp.local_prop_width, s);
-            launch_local<DIR_T2B>(A, cam, pcam, hp.local_prop_width, s);
-            if (prof.enabled) {
-                cudaEventRecord(prof.ev1, s);
-                cudaEventSynchronize(prof.ev1);
-                float ms = 0;
-                cudaEventElapsedTime(&ms, prof.ev0, prof.ev1);
-                prof.local_ms += ms, prof.local_runs++;
-            }
+            timed(prof, s, prof.local_ms, prof.local_runs, [&] {
+                launch_local<DIR_L2R>(A, cam, pcam, hp.local_prop_width, s);
+                launch_local<DIR_B2T>(A, cam, pcam, hp.local_prop_width, s);
+                launch_local<DIR_R2L>(A, cam, pcam, hp.local_prop_width, s);
+                launch_local<DIR_T2B>(A, cam, pcam, hp.local_prop_width, s);
+            });
         }
         VB_RETURN_IF_CUDA_ERROR();
     }
     A.rig = rig.ptr;  // the E-step writes the raw posteriors
-    {
-        KernelProfile none;
-        KernelProfile& prof = this->prof ? *this->prof : none;
-        if (prof.enabled) {
-            if (!prof.ev0) cudaEventCreate(&prof.ev0), cudaEventCreate(&prof.ev1);
-            cudaEventRecord(prof.ev0, s);
-        }
-        k_update_rigidness<<<pg, pb, 0, s>>>(A, cam, pcam);
-        if (prof.enabled) {
-            cudaEventRecord(prof.ev1, s);
-            cudaEventSynchronize(prof.ev1);
-            float ms = 0;
-            cudaEventElapsedTime(&ms, prof.ev0, prof.ev1);
-            prof.estep_ms += ms, prof.estep_launches++;
-        }
-    }
+    timed(prof, s, prof.estep_ms, prof.estep_launches, [&] { k_update_rigidness<<<pg, pb, 0, s>>>(A, cam, pcam); });
     VB_RETURN_IF_CUDA_ERROR();
     if (overlap_smoothing && hp.fb_smooth && N > 0) {
         // smooth the new rigidness maps for the next M-step on the side stream, concurrently with whatever the
@@ -1101,19 +921,8 @@ int DepthEM::run(int N, int N_dp, const DepthHyper& hp, bool update_rigidness_on
         StackView S{rig_s.ptr, rig_s.pitch, rig_s.layer_elems()};
         StackView F{fb_fwd.ptr, fb_fwd.pitch, fb_fwd.layer_elems()};
         StackView B{fb_bwd.ptr, fb_bwd.pitch, fb_bwd.layer_elems()};
-        {
-            KernelProfile none;
-            KernelProfile& prof = this->prof ? *this->prof : none;
-            if (prof.enabled) cudaEventRecord(prof.ev0, side);
-            fb_smooth_stack(E, S, F, B, N, w, h, hp.s0_ems_prob, hp.no_change_prob, side);
-            if (prof.enabled) {
-                cudaEventRecord(prof.ev1, side);
-                cudaEventSynchronize(prof.ev1);
-                float ms = 0;
-                cudaEventElapsedTime(&ms, prof.ev0, prof.ev1);
-                prof.smooth_ms += ms, prof.smooth_runs++;
-            }
-        }
+        timed(prof, side, prof.smooth_ms, prof.smooth_runs,
+              [&] { fb_smooth_stack(E, S, F, B, N, w, h, hp.s0_ems_prob, hp.no_change_prob, side); });
         VB_CUDA(cudaEventRecord(ev_smooth_done, side));
         smooth_layers = N, smooth_s0 = hp.s0_ems_prob, smooth_nc = hp.no_change_prob;
         VB_RETURN_IF_CUDA_ERROR();

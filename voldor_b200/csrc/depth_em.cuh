@@ -76,7 +76,7 @@ struct DepthEM {
 struct KernelProfile {
     bool enabled = false;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    double search_ms = 0;      // accumulated duration of k_cost_and_random_search
+    double search_ms = 0;      // accumulated duration of k_cost_and_random_search_pruned
     long long search_launches = 0;
     double estep_ms = 0;       // k_update_rigidness
     long long estep_launches = 0;
