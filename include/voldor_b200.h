@@ -55,8 +55,9 @@ int vb_align_frame_eval_gpu(int ref_fid, int tar_fid, const float* h_params_ref,
 
 /* No counterpart in the reference ABI: the same evaluation restricted to the samples its only caller reads — every
  * stride-th pixel in x and y (frame-alignment/align_frame_cost_fun.h:183-229), packed as
- * out[(y/stride) * ceil(w/stride) + x/stride] (x9 for the Jacobian).  stride 16 cuts the per-evaluation D2H from
- * 40 B/px to 40/256 B/px.  Values are those of vb_align_frame_eval_gpu at the same pixels. */
+ * out[(y/stride) * ceil(w/stride) + x/stride] (x9 for the Jacobian).  slam_py uses stride 4 for local links and 3 for
+ * loop closures, which cut the per-evaluation D2H from 40 B/px to 40/16 and 40/9 B/px.  Values are those of
+ * vb_align_frame_eval_gpu at the same pixels. */
 int vb_align_frame_eval_strided(int ref_fid, int tar_fid, const float* h_params_ref, const float* h_params_tar,
                                 float* h_o_residual, float* h_o_jacobian, int apply_weights, int stride);
 
@@ -71,7 +72,31 @@ int vb_py_voldor_wrapper(const float* flows, const float* disparity, const float
                          const char* config, int* n_registered, float* poses, float* poses_covar, float* depth,
                          float* depth_conf);
 
+/* reference: frame-alignment/py_export.h (py_export.cpp, align_frame.cpp) — keyframe alignment with the solver on
+ * the device (DESIGN.md §9).  Runs on the calling thread's execution context.  Returns 0, a CUDA error code, or: */
+#define VB_FALIGN_EINVAL (-1) /* N outside 2..64, stride < 1, connectivity entry out of range or unterminated */
+#define VB_FALIGN_EDEBUG (-2) /* debug != 0 (the reference opens OpenCV windows) */
+int vb_py_falign_wrapper(const float* depths, const float* images, const float* weights, const float* poses_init,
+                         float* poses_ret, const int* connectivity, float* poses_covar, float* scaling_factor,
+                         float* visibility_mat, float* consistency_mat, int N, int w, int h, float fx, float fy,
+                         float cx, float cy, float vbf, float crw, int optimize_7dof, int graduated_optmize, int stride,
+                         float consistency_residual_bound, int debug);
+
 /* ---- additions that have no counterpart in the reference ---- */
+
+/* Same alignment, also reporting what the solve did.  n_connectivity: length of `connectivity` in ints including
+ * the -1 terminator (< 0: scan to the terminator).  iters_run: LM iterations; reason: termination (1 gradient,
+ * 2 parameter, 3 function tolerance, 4 minimum trust-region radius, 5 iteration limit, 6 invalid steps);
+ * costs[2]: initial and final cost 1/2 sum f^2; stats[4] ms: total, upload + preparation, LM loop, covariance +
+ * scores + download.  samples (test hook, may be NULL): the per-sample residuals [pairs][n] and Jacobians
+ * [pairs][n][9] of the first evaluation, n = ceil(w/stride) * ceil(h/stride), as vb_align_frame_eval_strided
+ * packs them.  Any output pointer except the reference's may be NULL. */
+int vb_py_falign_wrapper_ex(const float* depths, const float* images, const float* weights, const float* poses_init,
+                            float* poses_ret, const int* connectivity, int n_connectivity, float* poses_covar,
+                            float* scaling_factor, float* visibility_mat, float* consistency_mat, int N, int w, int h,
+                            float fx, float fy, float cx, float cy, float vbf, float crw, int optimize_7dof,
+                            int graduated_optmize, int stride, float consistency_residual_bound, int debug,
+                            int* iters_run, int* reason, double* costs, float* stats, float* samples);
 
 /* Monocular bootstrap injection: when set (valid != 0), the next windows that have no depth prior start from
  * this pose (R row-major 3x3, t) and depth map instead of the essential-matrix bootstrap

@@ -10,5 +10,7 @@ _os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
 
 from .pyvoldor_vo import (voldor, load_library, set_bootstrap_override, voldor_ex, select_context,  # noqa: F401
                           context_srand, set_device)
+from .falign import falign, falign_ex  # noqa: F401,E402
 
-__all__ = ["voldor", "voldor_ex", "load_library", "set_bootstrap_override", "select_context", "context_srand", "set_device"]
+__all__ = ["voldor", "voldor_ex", "falign", "falign_ex", "load_library", "set_bootstrap_override", "select_context",
+           "context_srand", "set_device"]

@@ -17,6 +17,7 @@
 #include <mutex>
 #include <vector>
 #include "depth_em.cuh"
+#include "falign.cuh"
 #include "libc_rand.h"
 #include "pose_mode.cuh"
 #include "pose_sampler.cuh"
@@ -82,6 +83,7 @@ struct Context {
     AbiScratch abi;
     WindowScratch ws;
     BootstrapOverride boot;
+    FalignState fa;  // frame alignment (falign.cu); the reference-ABI align_frame_* entry points keep their own state
     std::unique_ptr<RandStream> rnd;
 
     explicit Context(int id_) : id(id_) {
